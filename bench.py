@@ -1,14 +1,18 @@
 #!/usr/bin/env python
 """bench.py -- env steps/sec of the Anakin ff_ppo training step (BASELINE.json metric) on N B200s.
 
-  python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun by the driver)
+  python bench.py --gpus N --steps K --warmup W            (N>1: launch under torchrun)
+  python bench.py ... --dump-outputs DIR                   also write the last timed step's outputs as DIR/<name>.npy
   python bench.py --impl reference ...                     CPU arm: the torch-CPU port of the same step
 
 One "step" = one Anakin update step per GPU: T=128 env steps of E=4096 envs (rollout with the
 actor/critic MLP[256,256] forwards on synthetic Box obs_dim=64 observations), the GAE scan, and
 4 epochs x 16 minibatches of the fused PPO loss/backward + clip/Adam (+ gradient all-reduce for N>1).
 value = N * T * E * K / time (whole-job env steps/s), timed with CUDA events on the stream the work
-runs on, barrier + synchronize on both sides, MAX over ranks.  Working set per step (trajectory obs +
+runs on, barrier + synchronize on both sides, MAX over ranks.  Two timed regions of K steps each run:
+the device-resident one (value) and the end-to-end one with host copies (e2e, with the spread over its
+K steps).  The inputs are seeded (arch.seed), so the same arguments give the same inputs on every
+run and the dumped outputs of two builds can be compared array for array.  Working set per step (trajectory obs +
 next_obs = 2 x 128 MiB fp32, or 2 x 64 MiB bf16) exceeds L2 together with weights/activations, so no
 explicit L2 flush is needed between steps (stated in config.l2).
 """
@@ -239,6 +243,37 @@ def _one_minibatch(model, tr, perm, i, mb):
 
 
 # ----------------------------------------------------------------------------------------------------
+def output_arrays(out):
+    """What one learn() call hands its caller (AnakinExperimentOutput), as float32 / float64 host arrays: the parameters
+    and Adam state of the learner state, the observation the next call starts from, and the episode / train metrics.
+    About 9 MB at the bench shape, so nothing needs sampling."""
+    import torch
+
+    ls = out.learner_state
+    host = lambda t, dt=torch.float32: t.detach().to("cpu", dt).numpy()
+    arrays = {"actor_params": host(ls.params.actor_params.flat), "critic_params": host(ls.params.critic_params.flat)}
+    for side, st in (("actor", ls.opt_states.actor_opt_state), ("critic", ls.opt_states.critic_opt_state)):
+        arrays[f"{side}_adam_mu"], arrays[f"{side}_adam_nu"] = host(st.mu), host(st.nu)
+        arrays[f"{side}_adam_count"], arrays[f"{side}_schedule_count"] = host(st.count, torch.float64), host(st.sched_count, torch.float64)
+    for u, ts in enumerate(ls.timestep):
+        arrays[f"next_observation_shard{u}"] = host(ts.observation)
+    for name, t in out.episode_metrics.items():
+        arrays[name] = host(t)
+    for name, t in out.train_metrics.items():
+        arrays[f"train_{name}"] = host(t)
+    return arrays
+
+
+def dump_outputs(arrays, directory):
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes exceed the 64 MiB budget"
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def run_ours(args):
     # Libraries (NCCL prints its version banner on stdout) must not pollute the ONE JSON line: everything
     # written to fd 1 during the run goes to stderr; the JSON line is written to the real stdout at the end.
@@ -317,18 +352,6 @@ def run_ours(args):
     dt = ev0.elapsed_time(ev1) * 1e-3
     progress(f"timed region A done {dt:.3f}s")
 
-    # ---- spread: the same K-step region nine more times (median / min / max beside the contract's single region) ----
-    region_ms = [dt / args.steps * 1e3]
-    for _ in range(9):
-        barrier()
-        a, b2 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        for _ in range(args.steps):
-            state = learn(state).learner_state
-        b2.record()
-        barrier()
-        region_ms.append(a.elapsed_time(b2) / args.steps)
-
     # ---- timed region B: end to end through the public API with host buffers (e2e) ----
     sh = learn.built["shards"][0]
     host_obs = torch.empty(sh.obs[T].shape, dtype=sh.obs.dtype).pin_memory()
@@ -339,9 +362,10 @@ def run_ours(args):
     h2d = host_obs.numel() * host_obs.element_size()
     d2h = host_train.numel() * 4 + host_ret.numel() * 4 + host_term.numel() + h2d  # + the carried observation
     barrier()
-    ev2, ev3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ev2.record()
-    for _ in range(args.steps):
+    # an event after every step (the stream is idle there, waiting for the host) gives the spread over the K steps
+    evs = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps + 1)]
+    evs[0].record()
+    for ev in evs[1:]:
         sh.obs[T].copy_(host_obs, non_blocking=True)      # H2D: the step's input observations (pinned)
         out = learn(state)
         state = out.learner_state
@@ -350,11 +374,14 @@ def run_ours(args):
         host_term.copy_(out.episode_metrics["is_terminal_step"][0, 0], non_blocking=True)
         torch.cuda.current_stream().synchronize()         # the host consumes the step's result
         host_obs.copy_(sh.obs[T])                         # D2H: the observation the next step starts from
-    ev3.record()
+        ev.record()
     barrier()
-    dt_e2e = ev2.elapsed_time(ev3) * 1e-3
+    dt_e2e = evs[0].elapsed_time(evs[-1]) * 1e-3
+    step_ms = [a.elapsed_time(b) for a, b in zip(evs, evs[1:])]
     clocks = sampler.stop()
     progress("timed region B done")
+    if args.dump_outputs and rank == 0:  # before the phase replays below move the learner state on
+        dump_outputs(output_arrays(out), args.dump_outputs)
 
     # ---- max over ranks ----
     times = torch.tensor([dt, dt_e2e], dtype=torch.float64, device="cuda")
@@ -441,11 +468,11 @@ def run_ours(args):
             "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "bf16" if precision == "bf16" else "f32", "data": "synthetic", "config": workload_config(world, precision),
             "e2e": {"value": e2e, "unit": "env_steps/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "ms_per_step": dt_e2e / args.steps * 1e3},
+                    "ms_per_step": dt_e2e / args.steps * 1e3,
+                    "ms_per_step_spread": {"steps": len(step_ms), "median": statistics.median(step_ms), "min": min(step_ms),
+                                           "max": max(step_ms)}},
             "gpu_launches": int(launches_per_update * args.steps), "launches_per_step": int(launches_per_update),
             "allreduce": ("none" if world == 1 else ("fused NVLink one-shot all-reduce inside the optimiser kernel" if learn.built.get("peers_obj") is not None else "NCCL all-reduce")),
-            "ms_per_step_spread": {"regions": len(region_ms), "median": statistics.median(region_ms), "min": min(region_ms),
-                                   "max": max(region_ms)},
             "clocks": clocks, "roofline": roofline, "gae_roofline": gae_roof, "phase_ms": phase_ms,
             "tensor_roofline_env_steps_per_s_per_gpu": peaks["bf16_tflops_sustained"] * 1e12 / sum(flops_per_env_step()),
         }
@@ -471,7 +498,10 @@ def main():
     ap.add_argument("--precision", default=os.environ.get("STX_BENCH_PRECISION", "bf16"), choices=["f32", "bf16"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--nccl-allreduce", action="store_true", help="N>1: NCCL all-reduce + K4 instead of the fused NVLink all-reduce/optimiser kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
